@@ -58,7 +58,15 @@ def parse_args():
     ap.add_argument("--no-other-mode", action="store_true", help="skip the secondary leg (the other plan mode)")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the bounded runs of BASELINE configs[2]-[4]")
     ap.add_argument("--cpu-sample", type=int, default=16, help="instances the CPU baseline explains")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/shap_values.npy (float64, "
+                         "[classes, instances of all ranks, groups]), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA engine (--impl ours)")
+    return args
 
 
 def workload(rank=0):
@@ -517,6 +525,12 @@ def run_ours(args):
     clocks = sampler.stop()
     engine.check_status()
     launches = engine.kernel_launches() - launches0
+    # what the last timed step handed its caller: this rank's phi block, or the gathered phi of every rank (N > 1)
+    if args.dump_outputs and rank == 0:
+        last_phi = (phi_dev if world == 1 else gather.buffer if gather is not None else phi_all).cpu().numpy()
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "shap_values.npy"),
+                last_phi.reshape(world, C, n, G).transpose(1, 0, 2, 3).reshape(C, world * n, G))
     # per-kernel device time (CUDA events around the coalition stage): three extra steps with plain launches -- the replayed
     # graph of the timed region carries no timing nodes
     engine.set_option("graph", 0)

@@ -30,11 +30,13 @@ def test_library_builds_and_exports_declared_symbols():
 
 
 def test_sass_is_sm100a():
-    if build.find_nvcc() is None:
+    nvcc = build.find_nvcc()
+    if nvcc is None:
         pytest.skip("no CUDA toolkit")
     import subprocess
     _cabi.load()
-    out = subprocess.run(["cuobjdump", "-lelf", build.LIB_PATH], capture_output=True, text=True).stdout
+    cuobjdump = os.path.join(os.path.dirname(nvcc), "cuobjdump")     # the toolkit's bin directory need not be on PATH
+    out = subprocess.run([cuobjdump, "-lelf", build.LIB_PATH], capture_output=True, text=True).stdout
     assert "sm_100a" in out
 
 
