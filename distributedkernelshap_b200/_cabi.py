@@ -44,6 +44,8 @@ SIGNATURES = {
     "dks_set_background": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "dks_set_groups": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "dks_set_model": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_double, C.c_int]),
+    "dks_set_mlp_model": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                    C.c_double, C.c_int]),
     "dks_set_link": (C.c_int, [C.c_void_p, C.c_int]),
     "dks_fit": (C.c_int, [C.c_void_p]),
     "dks_num_outputs": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),

@@ -11,6 +11,7 @@
 #include "dks_l1.cuh"
 #include "dks_wide.cuh"
 #include "dks_sampler.cuh"
+#include "dks_mlp.cuh"
 
 namespace {
 
@@ -87,7 +88,7 @@ int bind(dks_ctx* ctx) {
 int ensure_workspace(dks_ctx* ctx, int n) {
     if (n <= ctx->cap_n) return DKS_OK;
     const int G = ctx->G, R = ctx->R, C = ctx->C;
-    TRY(dev_alloc(&ctx->d_XW, (size_t)n * G * R));
+    TRY(dev_alloc(&ctx->d_XW, (size_t)n * G * (ctx->mlp ? ctx->H : R)));
     TRY(dev_alloc(&ctx->d_XT, (size_t)n * ((G + 3) / 4) * 16));
     TRY(dev_alloc(&ctx->d_vflag, (size_t)n * G));
     TRY(dev_alloc(&ctx->d_vmask, (size_t)n));
@@ -122,6 +123,20 @@ int launch_prepare(dks_ctx* ctx, const double* X_dev, int n) {
     CUDA_TRY(cudaMemsetAsync(ctx->d_status, 0, sizeof(int) * (4 + G + 1), ctx->stream));
     if (!ctx->capturing) ctx->last_was_graph = false;
     CUDA_TRY(record_ev(ctx, 0));
+    if (ctx->mlp) {
+        dks::mlp::mlp_prep_kernel<<<n, 128, 0, ctx->stream>>>(
+            X_dev, ctx->d_W, ctx->d_b, ctx->d_W2, ctx->d_b2, ctx->d_bg, ctx->d_goff, ctx->d_gcols, ctx->d_colmin,
+            ctx->d_colmax, ctx->d_colnan, ctx->d_linkfnull, n, ctx->N, ctx->D, G, ctx->H, ctx->R, ctx->C, ctx->act, ctx->kappa,
+            ctx->link, ctx->d_XW, ctx->d_vmask, ctx->d_M, ctx->d_dlink, ctx->d_hist, ctx->d_counts, ctx->d_idx_full,
+            ctx->d_idx_other);
+        ctx->launches += 1;
+        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(record_ev(ctx, 1));
+        ctx->cur_n = n;
+        ctx->cur_X = X_dev;
+        ctx->prepared = true;
+        return DKS_OK;
+    }
     int ipb = 256 / G;
     if (ipb < 1) ipb = 1;
     const bool stage = dks::prep_smem_bytes(true, ipb, G, ctx->R, ctx->D) <= (size_t)96 * 1024;
@@ -139,6 +154,202 @@ int launch_prepare(dks_ctx* ctx, const double* X_dev, int n) {
     ctx->cur_n = n;
     ctx->cur_X = X_dev;
     ctx->prepared = true;
+    return DKS_OK;
+}
+
+// the solve behind the shared-plan coalition kernels: from the (sum p1, sum p0) buffer of the instances whose groups all
+// vary to phi (projection solve, normal-matrix solve, l1 selection, or the float64 product beyond 128 groups)
+int launch_sums_solve(dks_ctx* ctx, const PlanDev& pg, int n, double* phi_dev, bool l1) {
+    const int G = ctx->G, S = pg.S, S_pad = pg.S_pad;
+    dks::shared_path::WlsSharedParams wp;
+    wp.n = n; wp.N = ctx->N; wp.G = G; wp.C = ctx->C; wp.S = S; wp.S_pad = S_pad; wp.link = ctx->link;
+    wp.uniform_w = 1; wp.sums = ctx->d_sums; wp.z = pg.z; wp.w = pg.w; wp.ainv = pg.ainv; wp.dlink = ctx->d_dlink;
+    wp.linkfnull = ctx->d_linkfnull; wp.fnull = ctx->d_fnull; wp.list = ctx->d_idx_full; wp.count = ctx->d_counts;
+    wp.phi = phi_dev;
+    if (l1) {
+        // upstream's l1 branch: moments of y per instance, then the LARS path + criterion + restricted WLS, one warp each
+        const dks_ctx::L1Dev& lt = ctx->h_l1[G];
+        const size_t need_m = (size_t)n * (2 * G + 4);
+        if (need_m > ctx->cap_mom) { TRY(dev_alloc(&ctx->d_mom, need_m)); ctx->cap_mom = need_m; ctx->epoch++; }
+        dks::l1::Params lp;
+        memset(&lp, 0, sizeof(lp));
+        lp.n = n; lp.N = ctx->N; lp.G = G; lp.C = ctx->C; lp.S = S; lp.S_pad = S_pad; lp.link = ctx->link;
+        lp.mode = ctx->l1_mode; lp.kfeat = ctx->l1_k; lp.sums = ctx->d_sums; lp.z = pg.z; lp.w = pg.w;
+        lp.t.gram_raw = lt.gram_raw; lp.t.gram_norm = lt.gram_norm; lp.t.colsum = lt.colsum; lp.t.scale = lt.scale;
+        lp.t.bz = lt.bz; lp.t.gram_w = lt.gram_w; lp.t.b = lt.b; lp.t.sqab = lt.sqab; lp.t.sum_b = lt.sum_b;
+        lp.t.sum_sqb = lt.sum_sqb; lp.t.n_aug = lt.n_aug;
+        lp.dlink = ctx->d_dlink; lp.linkfnull = ctx->d_linkfnull; lp.fnull = ctx->d_fnull; lp.list = ctx->d_idx_full;
+        lp.count = ctx->d_counts; lp.mom = ctx->d_mom; lp.phi = phi_dev; lp.status = ctx->d_status;
+        const size_t msm = sizeof(double) * (size_t)S;
+        if (msm + 8192 > (size_t)ctx->max_smem_optin)
+            return fail(DKS_ERR_UNSUPPORTED, "l1 feature selection: %d coalitions per plan exceed the shared-memory staging", S);
+        const int mgrid = n < ctx->sm_count * 2 ? n : ctx->sm_count * 2;
+        if (pg.W == 1) {
+            CUDA_TRY(cudaFuncSetAttribute(dks::l1::l1_moments_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msm));
+            dks::l1::l1_moments_kernel<1><<<mgrid, dks::l1::MOM_THREADS, msm, ctx->stream>>>(lp);
+        } else {
+            CUDA_TRY(cudaFuncSetAttribute(dks::l1::l1_moments_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msm));
+            dks::l1::l1_moments_kernel<2><<<mgrid, dks::l1::MOM_THREADS, msm, ctx->stream>>>(lp);
+        }
+        const size_t per_warp = dks::l1::lars_smem_per_warp(G);
+        const size_t gram_bytes = sizeof(double) * (size_t)G * G;
+        const size_t budget = (size_t)ctx->max_smem_optin - 2048;
+        // the Gram matrix of the path goes to shared memory when at least four warps still fit next to it
+        const int stage_gram = (gram_bytes + 4 * per_warp <= budget) ? 1 : 0;
+        int wpc = (int)((budget - (stage_gram ? gram_bytes : 0)) / per_warp);
+        if (wpc < 1) return fail(DKS_ERR_UNSUPPORTED, "l1 feature selection: the %d x %d Cholesky factor does not fit shared memory", G, G);
+        if (wpc > 8) wpc = 8;
+        const size_t lsm = per_warp * wpc + (stage_gram ? gram_bytes : 0);
+        int per_sm = (int)((size_t)ctx->max_smem_optin / (lsm + 1024));
+        if (per_sm < 1) per_sm = 1;
+        if (per_sm > 4) per_sm = 4;
+        int lgrid = (n + wpc - 1) / wpc;
+        if (lgrid > ctx->sm_count * per_sm) lgrid = ctx->sm_count * per_sm;
+        CUDA_TRY(cudaFuncSetAttribute(dks::l1::l1_lars_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lsm));
+        dks::l1::l1_lars_kernel<<<lgrid, 32 * wpc, lsm, ctx->stream>>>(lp, wpc, stage_gram);
+    } else if (pg.W > 2) {
+        // more than 128 groups: link, float64 product with the host-supplied projection, remainder (dks_wide.cuh)
+        const size_t need_y = (size_t)n * S_pad, need_b = (size_t)n * pg.kpw;
+        if (need_y > ctx->cap_yw) { TRY(dev_alloc(&ctx->d_yw, need_y)); ctx->cap_yw = need_y; ctx->epoch++; }
+        if (need_b > ctx->cap_betaw) { TRY(dev_alloc(&ctx->d_betaw, need_b)); ctx->cap_betaw = need_b; ctx->epoch++; }
+        dks::wide::WideParams qp;
+        memset(&qp, 0, sizeof(qp));
+        qp.n = n; qp.N = ctx->N; qp.G = G; qp.C = ctx->C; qp.S = S; qp.S_pad = S_pad; qp.KP = pg.kpw; qp.link = ctx->link;
+        qp.sums = ctx->d_sums; qp.PT = pg.ptw; qp.dvec = pg.dvecw; qp.dlink = ctx->d_dlink;
+        qp.linkfnull = ctx->d_linkfnull; qp.fnull = ctx->d_fnull; qp.list = ctx->d_idx_full; qp.count = ctx->d_counts;
+        qp.y = ctx->d_yw; qp.beta = ctx->d_betaw; qp.phi = phi_dev;
+        CUDA_TRY(dks::wide::launch_wide_solve(qp, n, ctx->sm_count, ctx->opt_wide_gemm, ctx->stream));
+        ctx->launches += 2;                      // three launches; the common tail below counts one of them
+    } else if (pg.pmat != nullptr) {
+        dks::shared_path::WlsPmatParams pp;
+        pp.n = n; pp.N = ctx->N; pp.G = G; pp.C = ctx->C; pp.S = S; pp.S_pad = S_pad; pp.link = ctx->link; pp.uniform_w = 1;
+        pp.sums = ctx->d_sums; pp.pmat = pg.pmat; pp.dvec = pg.dvec; pp.dlink = ctx->d_dlink;
+        pp.linkfnull = ctx->d_linkfnull; pp.fnull = ctx->d_fnull; pp.list = ctx->d_idx_full; pp.count = ctx->d_counts;
+        pp.phi = phi_dev;
+        cudaError_t perr = cudaSuccess;
+        if (!dks::shared_path::launch_wls_pmat(pp, n, ctx->sm_count, ctx->max_smem_optin, ctx->stream, &perr))
+            return fail(DKS_ERR_UNSUPPORTED, "projection solve does not fit shared memory");
+        CUDA_TRY(perr);
+    } else {
+        const size_t wsm = dks::shared_path::wls_shared_smem(G);
+        int per_sm = (int)((size_t)ctx->max_smem_optin / (wsm + 24 * 1024));
+        if (per_sm > 4) per_sm = 4;
+        if (per_sm < 1) per_sm = 1;
+        int wgrid = n < ctx->sm_count * per_sm ? n : ctx->sm_count * per_sm;   // persistent CTAs of 8 warps
+        if (pg.W == 1) {
+            CUDA_TRY(cudaFuncSetAttribute(dks::shared_path::wls_shared_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsm));
+            dks::shared_path::wls_shared_kernel<1><<<wgrid, dks::shared_path::WLS_THREADS, wsm, ctx->stream>>>(wp);
+        } else {
+            CUDA_TRY(cudaFuncSetAttribute(dks::shared_path::wls_shared_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsm));
+            dks::shared_path::wls_shared_kernel<2><<<wgrid, dks::shared_path::WLS_THREADS, wsm, ctx->stream>>>(wp);
+        }
+    }
+    return DKS_OK;
+}
+
+// Coalition stage of a one-hidden-layer ReLU network (dks_mlp.cuh): the shared-plan MLP kernel for the instances whose
+// groups all vary (binary head, uniform background weights, the engine's plans), then the linear engine's solve of its
+// (sum p1, sum p0) buffer; the general MLP kernel for everything else.  No linear coalition kernel runs on such a context.
+int launch_explain_mlp(dks_ctx* ctx, ExplainParams& p, double* phi_dev, bool ext) {
+    const int n = ctx->cur_n, G = ctx->G;
+    const int kernel = ctx->kernel_choice;
+    if (kernel == DKS_KERNEL_TCGEN05)
+        return fail(DKS_ERR_UNSUPPORTED, "the tcgen05 kernel evaluates linear models only (this context holds an MLP)");
+    dks::mlp::GenParams gp;
+    gp.H = ctx->H; gp.BW1 = ctx->d_BW; gp.base1 = ctx->d_scores; gp.W2 = ctx->d_W2; gp.b2 = ctx->d_b2;
+    const PlanDev& pg = ctx->h_plans[G];
+    const bool fast = (kernel == DKS_KERNEL_AUTO || kernel == DKS_KERNEL_SHARED) && !ext && ctx->act == DKS_ACT_BINARY_LOGISTIC &&
+                      ctx->uniform_w && G >= 2 && pg.mlp_dT != nullptr && pg.S == dks_effective_S(G, ctx->nsamples_req);
+    if (kernel == DKS_KERNEL_SHARED && !fast && !ext && pg.z != nullptr)
+        return fail(DKS_ERR_UNSUPPORTED, "shared-plan MLP kernel needs the binary-logistic head, uniform background weights, "
+                    "at most %d hidden units after sign padding and at most %d background rows", dks::mlp::MAX_H,
+                    dks::mlp::FAST_MAXN);
+    const bool l1 = ctx->l1_mode != 0;
+    if (l1) {
+        if (ext || ctx->plan_mode == 1) return fail(DKS_ERR_UNSUPPORTED, "l1 feature selection runs on shared plans only");
+        if (!fast || ctx->h_l1[G].gram_raw == nullptr || ctx->h_l1[G].S != pg.S)
+            return fail(DKS_ERR_UNSUPPORTED, "l1 feature selection needs the shared-plan path (binary-logistic head, uniform "
+                        "background weights) and the l1 tables of the M=%d plan (dks_set_l1_tables)", G);
+    }
+    cudaStream_t gstream = ctx->stream;
+    if (fast && ctx->side_stream != nullptr) {
+        CUDA_TRY(cudaEventRecord(ctx->ev_fork, ctx->stream));
+        CUDA_TRY(cudaStreamWaitEvent(ctx->side_stream, ctx->ev_fork, 0));
+        gstream = ctx->side_stream;
+    }
+    auto join = [&]() -> cudaError_t {
+        if (gstream == ctx->stream) return cudaSuccess;
+        cudaError_t e = cudaEventRecord(ctx->ev_join, gstream);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0);
+        return e;
+    };
+    if (fast) {
+        const int S = pg.S, S_pad = pg.S_pad, HP = ctx->mlp_hp;
+        const size_t need = (size_t)n * S_pad;
+        if (need > ctx->cap_sums) { TRY(dev_alloc(&ctx->d_sums, need)); ctx->cap_sums = need; ctx->epoch++; }
+        // a'(q, s, u) goes through a workspace of at most 1 GiB: chunks of QC instances
+        const size_t per_inst = (size_t)S_pad * HP;
+        int QC = (int)(((size_t)1 << 28) / per_inst) / 32 * 32;
+        if (QC < 32) QC = 32;
+        if (QC > (n + 31) / 32 * 32) QC = (n + 31) / 32 * 32;
+        const size_t need_a = (size_t)QC * per_inst;
+        if (need_a > ctx->cap_mlp_atab) { TRY(dev_alloc(&ctx->d_mlp_atab, need_a)); ctx->cap_mlp_atab = need_a; ctx->epoch++; }
+        dks::mlp::SharedParams sp;
+        memset(&sp, 0, sizeof(sp));
+        sp.N = ctx->N; sp.G = G; sp.H = ctx->H; sp.HP = HP; sp.S = S; sp.S_pad = S_pad; sp.QC = QC;
+        sp.scale = ctx->scale; sp.b2 = ctx->h_b2[0]; sp.negmask = ctx->mlp_negmask;
+        sp.dT = pg.mlp_dT; sp.Ld = pg.mlp_Ld; sp.z = pg.z; sp.XW = ctx->d_XW; sp.perm = ctx->d_mlp_perm;
+        sp.w2abs = ctx->d_mlp_w2abs; sp.atab = ctx->d_mlp_atab; sp.list = ctx->d_idx_full; sp.count = ctx->d_counts;
+        sp.sums = ctx->d_sums;
+        const size_t asm_bytes = sizeof(float) * (size_t)G * HP;
+        const size_t ssm = dks::mlp::shared_smem_bytes(ctx->N, HP);
+        CUDA_TRY(cudaFuncSetAttribute(dks::mlp::mlp_atab_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)asm_bytes));
+        auto skern = dks::mlp::mlp_shared_kernel<16>;
+        switch (HP) {
+            case 16: skern = dks::mlp::mlp_shared_kernel<16>; break;
+            case 32: skern = dks::mlp::mlp_shared_kernel<32>; break;
+            case 48: skern = dks::mlp::mlp_shared_kernel<48>; break;
+            case 64: skern = dks::mlp::mlp_shared_kernel<64>; break;
+            case 80: skern = dks::mlp::mlp_shared_kernel<80>; break;
+            case 96: skern = dks::mlp::mlp_shared_kernel<96>; break;
+            case 112: skern = dks::mlp::mlp_shared_kernel<112>; break;
+            case 128: skern = dks::mlp::mlp_shared_kernel<128>; break;
+            default: return fail(DKS_ERR_INVALID, "MLP unit order of %d units", HP);
+        }
+        CUDA_TRY(cudaFuncSetAttribute(skern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ssm));
+        for (int q0 = 0; q0 < n; q0 += QC) {
+            sp.q0 = q0;
+            dks::mlp::mlp_atab_kernel<<<QC, 256, asm_bytes, ctx->stream>>>(sp);
+            skern<<<S, 128, ssm, ctx->stream>>>(sp);
+            ctx->launches += 2;
+        }
+        CUDA_TRY(cudaGetLastError());
+        TRY(launch_sums_solve(ctx, pg, n, phi_dev, l1));
+        ctx->launches += 1;
+        CUDA_TRY(cudaGetLastError());
+        p.list = ctx->d_idx_other;      // the general kernel below takes the remaining instances
+        p.count = ctx->d_counts + 1;
+    }
+    if (l1 && !ctx->l1_others_plain) {
+        // instances with a partial varying set would need their own selection: reported, not computed
+        dks::flag_unsupported_kernel<<<1, 1, 0, gstream>>>(ctx->d_counts + 1, G, ctx->d_status);
+    } else {
+        const int nacc = dks::mlp::gen_nacc(ctx->act, ctx->C);
+        const size_t smem = dks::mlp::gen_smem_bytes(p.S_cap, G < 64 ? G : 64, ctx->R, nacc);
+        if ((long long)smem > (long long)ctx->max_smem_optin)
+            return fail(DKS_ERR_UNSUPPORTED, "general MLP kernel needs %zu B of shared memory (> %d): nsamples too large", smem,
+                        ctx->max_smem_optin);
+        CUDA_TRY(cudaFuncSetAttribute(dks::mlp::mlp_general_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        int per_sm = (int)((size_t)ctx->max_smem_optin / (smem + 1024));
+        if (per_sm < 1) per_sm = 1;
+        if (per_sm > 8) per_sm = 8;
+        int grid = ctx->sm_count * per_sm;
+        if (grid > n) grid = n;
+        dks::mlp::mlp_general_kernel<<<grid, dks::mlp::GEN_THREADS, smem, gstream>>>(p, gp);
+    }
+    ctx->launches += 1;
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(join());
     return DKS_OK;
 }
 
@@ -248,6 +459,11 @@ int launch_explain(dks_ctx* ctx, double* phi_dev, const uint64_t* ext_z, const d
 
     int kernel = ctx->kernel_choice;
     CUDA_TRY(record_ev(ctx, 2));
+    if (ctx->mlp) {
+        TRY(launch_explain_mlp(ctx, p, phi_dev, ext_z != nullptr));
+        CUDA_TRY(record_ev(ctx, 3));
+        return DKS_OK;
+    }
 
     // ---- shared-plan fast path: instances whose varying set is all G groups, evaluated against the plan's Dm table
     const int G = ctx->G;
@@ -328,89 +544,7 @@ int launch_explain(dks_ctx* ctx, double* phi_dev, const uint64_t* ext_z, const d
             sp.acache = ctx->d_acache;
         }
         ctx->launches += dks::shared_path::launch_explain_shared(sp, pg.W, ctx->sm_count, ctx->stream) - 1;
-        dks::shared_path::WlsSharedParams wp;
-        wp.n = n; wp.N = ctx->N; wp.G = G; wp.C = ctx->C; wp.S = S; wp.S_pad = S_pad; wp.link = ctx->link;
-        wp.uniform_w = 1; wp.sums = ctx->d_sums; wp.z = pg.z; wp.w = pg.w; wp.ainv = pg.ainv; wp.dlink = ctx->d_dlink;
-        wp.linkfnull = ctx->d_linkfnull; wp.fnull = ctx->d_fnull; wp.list = ctx->d_idx_full; wp.count = ctx->d_counts;
-        wp.phi = phi_dev;
-        if (l1) {
-            // upstream's l1 branch: moments of y per instance, then the LARS path + criterion + restricted WLS, one warp each
-            const dks_ctx::L1Dev& lt = ctx->h_l1[G];
-            const size_t need_m = (size_t)n * (2 * G + 4);
-            if (need_m > ctx->cap_mom) { TRY(dev_alloc(&ctx->d_mom, need_m)); ctx->cap_mom = need_m; ctx->epoch++; }
-            dks::l1::Params lp;
-            memset(&lp, 0, sizeof(lp));
-            lp.n = n; lp.N = ctx->N; lp.G = G; lp.C = ctx->C; lp.S = S; lp.S_pad = S_pad; lp.link = ctx->link;
-            lp.mode = ctx->l1_mode; lp.kfeat = ctx->l1_k; lp.sums = ctx->d_sums; lp.z = pg.z; lp.w = pg.w;
-            lp.t.gram_raw = lt.gram_raw; lp.t.gram_norm = lt.gram_norm; lp.t.colsum = lt.colsum; lp.t.scale = lt.scale;
-            lp.t.bz = lt.bz; lp.t.gram_w = lt.gram_w; lp.t.b = lt.b; lp.t.sqab = lt.sqab; lp.t.sum_b = lt.sum_b;
-            lp.t.sum_sqb = lt.sum_sqb; lp.t.n_aug = lt.n_aug;
-            lp.dlink = ctx->d_dlink; lp.linkfnull = ctx->d_linkfnull; lp.fnull = ctx->d_fnull; lp.list = ctx->d_idx_full;
-            lp.count = ctx->d_counts; lp.mom = ctx->d_mom; lp.phi = phi_dev; lp.status = ctx->d_status;
-            const size_t msm = sizeof(double) * (size_t)S;
-            if (msm + 8192 > (size_t)ctx->max_smem_optin)
-                return fail(DKS_ERR_UNSUPPORTED, "l1 feature selection: %d coalitions per plan exceed the shared-memory staging", S);
-            const int mgrid = n < ctx->sm_count * 2 ? n : ctx->sm_count * 2;
-            if (pg.W == 1) {
-                CUDA_TRY(cudaFuncSetAttribute(dks::l1::l1_moments_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msm));
-                dks::l1::l1_moments_kernel<1><<<mgrid, dks::l1::MOM_THREADS, msm, ctx->stream>>>(lp);
-            } else {
-                CUDA_TRY(cudaFuncSetAttribute(dks::l1::l1_moments_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msm));
-                dks::l1::l1_moments_kernel<2><<<mgrid, dks::l1::MOM_THREADS, msm, ctx->stream>>>(lp);
-            }
-            const size_t per_warp = dks::l1::lars_smem_per_warp(G);
-            const size_t gram_bytes = sizeof(double) * (size_t)G * G;
-            const size_t budget = (size_t)ctx->max_smem_optin - 2048;
-            // the Gram matrix of the path goes to shared memory when at least four warps still fit next to it
-            const int stage_gram = (gram_bytes + 4 * per_warp <= budget) ? 1 : 0;
-            int wpc = (int)((budget - (stage_gram ? gram_bytes : 0)) / per_warp);
-            if (wpc < 1) return fail(DKS_ERR_UNSUPPORTED, "l1 feature selection: the %d x %d Cholesky factor does not fit shared memory", G, G);
-            if (wpc > 8) wpc = 8;
-            const size_t lsm = per_warp * wpc + (stage_gram ? gram_bytes : 0);
-            int per_sm = (int)((size_t)ctx->max_smem_optin / (lsm + 1024));
-            if (per_sm < 1) per_sm = 1;
-            if (per_sm > 4) per_sm = 4;
-            int lgrid = (n + wpc - 1) / wpc;
-            if (lgrid > ctx->sm_count * per_sm) lgrid = ctx->sm_count * per_sm;
-            CUDA_TRY(cudaFuncSetAttribute(dks::l1::l1_lars_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lsm));
-            dks::l1::l1_lars_kernel<<<lgrid, 32 * wpc, lsm, ctx->stream>>>(lp, wpc, stage_gram);
-        } else if (pg.W > 2) {
-            // more than 128 groups: link, float64 product with the host-supplied projection, remainder (dks_wide.cuh)
-            const size_t need_y = (size_t)n * S_pad, need_b = (size_t)n * pg.kpw;
-            if (need_y > ctx->cap_yw) { TRY(dev_alloc(&ctx->d_yw, need_y)); ctx->cap_yw = need_y; ctx->epoch++; }
-            if (need_b > ctx->cap_betaw) { TRY(dev_alloc(&ctx->d_betaw, need_b)); ctx->cap_betaw = need_b; ctx->epoch++; }
-            dks::wide::WideParams qp;
-            memset(&qp, 0, sizeof(qp));
-            qp.n = n; qp.N = ctx->N; qp.G = G; qp.C = ctx->C; qp.S = S; qp.S_pad = S_pad; qp.KP = pg.kpw; qp.link = ctx->link;
-            qp.sums = ctx->d_sums; qp.PT = pg.ptw; qp.dvec = pg.dvecw; qp.dlink = ctx->d_dlink;
-            qp.linkfnull = ctx->d_linkfnull; qp.fnull = ctx->d_fnull; qp.list = ctx->d_idx_full; qp.count = ctx->d_counts;
-            qp.y = ctx->d_yw; qp.beta = ctx->d_betaw; qp.phi = phi_dev;
-            CUDA_TRY(dks::wide::launch_wide_solve(qp, n, ctx->sm_count, ctx->opt_wide_gemm, ctx->stream));
-            ctx->launches += 2;                      // three launches; the common tail below counts one of them
-        } else if (pg.pmat != nullptr) {
-            dks::shared_path::WlsPmatParams pp;
-            pp.n = n; pp.N = ctx->N; pp.G = G; pp.C = ctx->C; pp.S = S; pp.S_pad = S_pad; pp.link = ctx->link; pp.uniform_w = 1;
-            pp.sums = ctx->d_sums; pp.pmat = pg.pmat; pp.dvec = pg.dvec; pp.dlink = ctx->d_dlink;
-            pp.linkfnull = ctx->d_linkfnull; pp.fnull = ctx->d_fnull; pp.list = ctx->d_idx_full; pp.count = ctx->d_counts;
-            pp.phi = phi_dev;
-            cudaError_t perr = cudaSuccess;
-            if (!dks::shared_path::launch_wls_pmat(pp, n, ctx->sm_count, ctx->max_smem_optin, ctx->stream, &perr))
-                return fail(DKS_ERR_UNSUPPORTED, "projection solve does not fit shared memory");
-            CUDA_TRY(perr);
-        } else {
-            const size_t wsm = dks::shared_path::wls_shared_smem(G);
-            int per_sm = (int)((size_t)ctx->max_smem_optin / (wsm + 24 * 1024));
-            if (per_sm > 4) per_sm = 4;
-            if (per_sm < 1) per_sm = 1;
-            int wgrid = n < ctx->sm_count * per_sm ? n : ctx->sm_count * per_sm;   // persistent CTAs of 8 warps
-            if (pg.W == 1) {
-                CUDA_TRY(cudaFuncSetAttribute(dks::shared_path::wls_shared_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsm));
-                dks::shared_path::wls_shared_kernel<1><<<wgrid, dks::shared_path::WLS_THREADS, wsm, ctx->stream>>>(wp);
-            } else {
-                CUDA_TRY(cudaFuncSetAttribute(dks::shared_path::wls_shared_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsm));
-                dks::shared_path::wls_shared_kernel<2><<<wgrid, dks::shared_path::WLS_THREADS, wsm, ctx->stream>>>(wp);
-            }
-        }
+        TRY(launch_sums_solve(ctx, pg, n, phi_dev, l1));
         ctx->launches += 2;
         CUDA_TRY(cudaGetLastError());
         p.list = ctx->d_idx_other;      // the general kernel below takes the remaining instances
@@ -555,6 +689,8 @@ int dks_destroy(dks_ctx* ctx) {
     dev_free(&ctx->d_idx_full); dev_free(&ctx->d_idx_other); dev_free(&ctx->d_sums); dev_free(&ctx->d_acc); dev_free(&ctx->d_done); dev_free(&ctx->d_mom); dev_free(&ctx->d_step); dev_free(&ctx->d_peer_list);
     dev_free(&ctx->d_status); ctx->d_hist = nullptr; ctx->d_counts = nullptr; dev_free(&ctx->d_yw); dev_free(&ctx->d_betaw); dev_free(&ctx->d_acache); dev_free(&ctx->d_phi); if (ctx->h_phi_pin) { cudaFreeHost(ctx->h_phi_pin); ctx->h_phi_pin = nullptr; } dev_free(&ctx->d_genz); dev_free(&ctx->d_genw); dev_free(&ctx->d_genchol); dev_free(&ctx->d_genainv); dev_free(&ctx->d_afix); dev_free(&ctx->d_sinfo); dev_free(&ctx->d_extz);
     dev_free(&ctx->d_extw);
+    dev_free(&ctx->d_W2); dev_free(&ctx->d_b2); dev_free(&ctx->d_mlp_perm); dev_free(&ctx->d_mlp_w2abs);
+    dev_free(&ctx->d_mlp_atab);
     dev_free(&ctx->dbg_T);
     dev_free(&ctx->dbg_time);
     free_plan_allocs(ctx, -1);
@@ -636,6 +772,58 @@ int dks_set_model(dks_ctx* ctx, const double* W_host, const double* b_host, int 
     ctx->R = R; ctx->act = activation; ctx->kappa = kappa; ctx->scalar_out = scalar_out;
     ctx->h_W.assign(W_host, W_host + (size_t)R * ctx->D);
     ctx->h_b.assign(b_host, b_host + R);
+    ctx->mlp = false;
+    ctx->fitted = false;
+    return DKS_OK;
+}
+
+int dks_set_mlp_model(dks_ctx* ctx, const double* W1_host, const double* b1_host, int H, const double* W2_host,
+                      const double* b2_host, int R, int activation, double kappa, int scalar_out) {
+    BIND(ctx);
+    REQUIRE(ctx->D > 0, "dks_set_mlp_model: call dks_set_background first (D unknown)");
+    REQUIRE(W1_host && b1_host && W2_host && b2_host && H > 0 && R > 0, "dks_set_mlp_model: need W1, b1, W2, b2, H > 0, R > 0");
+    if (H > dks::mlp::MAX_H) return fail(DKS_ERR_UNSUPPORTED, "dks_set_mlp_model: H=%d hidden units; at most %d supported", H,
+                                         dks::mlp::MAX_H);
+    if (R > 8) return fail(DKS_ERR_UNSUPPORTED, "dks_set_mlp_model: R=%d output units; at most 8 supported", R);
+    int C = R;
+    if (activation == DKS_ACT_BINARY_LOGISTIC) {
+        REQUIRE(R == 1, "binary-logistic head needs R == 1 (got %d)", R);
+        REQUIRE(kappa > 0, "binary-logistic head needs kappa > 0");
+        C = 2;
+    } else if (activation == DKS_ACT_SOFTMAX) {
+        REQUIRE(R >= 2, "softmax head needs at least two output units (got %d)", R);
+    } else if (activation != DKS_ACT_IDENTITY) {
+        return fail(DKS_ERR_INVALID, "dks_set_mlp_model: unknown activation %d", activation);
+    }
+    ctx->C = C; ctx->R = R; ctx->H = H; ctx->act = activation; ctx->kappa = kappa; ctx->scalar_out = scalar_out;
+    ctx->h_W.assign(W1_host, W1_host + (size_t)H * ctx->D);
+    ctx->h_b.assign(b1_host, b1_host + H);
+    ctx->h_W2.assign(W2_host, W2_host + (size_t)R * H);
+    ctx->h_b2.assign(b2_host, b2_host + R);
+    // unit order of the shared-plan kernel (binary head): positive W2 first, then negative, each padded to whole chunks
+    ctx->mlp_hp = 0; ctx->mlp_negmask = 0;
+    ctx->h_mlp_perm.clear(); ctx->h_mlp_w2abs.clear();
+    if (R == 1) {
+        const int CH = dks::mlp::CHUNK;
+        std::vector<int> pos, neg;
+        for (int u = 0; u < H; ++u) {
+            if (W2_host[u] > 0) pos.push_back(u);
+            else if (W2_host[u] < 0) neg.push_back(u);
+        }
+        const int np = (int)(pos.size() + CH - 1) / CH * CH, nn = (int)(neg.size() + CH - 1) / CH * CH;
+        const int hp = (np + nn + 15) / 16 * 16;
+        if (hp >= 16 && hp <= dks::mlp::MAX_H) {
+            ctx->h_mlp_perm.assign(hp, -1);
+            ctx->h_mlp_w2abs.assign(hp, 0.f);
+            for (size_t k = 0; k < pos.size(); ++k) { ctx->h_mlp_perm[k] = pos[k]; ctx->h_mlp_w2abs[k] = (float)W2_host[pos[k]]; }
+            for (size_t k = 0; k < neg.size(); ++k) {
+                ctx->h_mlp_perm[np + k] = neg[k]; ctx->h_mlp_w2abs[np + k] = (float)-W2_host[neg[k]];
+            }
+            for (int c = np / CH; c < (np + nn) / CH; ++c) ctx->mlp_negmask |= 1u << c;
+            ctx->mlp_hp = hp;
+        }
+    }
+    ctx->mlp = true;
     ctx->fitted = false;
     return DKS_OK;
 }
@@ -662,6 +850,9 @@ int dks_fit(dks_ctx* ctx) {
         for (int c = 0; c < D; ++c) ctx->h_gcols[c] = c;
     }
     const int G = ctx->G;
+    if (ctx->mlp && G > 64)
+        return fail(DKS_ERR_UNSUPPORTED, "dks_fit: %d groups; networks are explained over at most 64 groups", G);
+    const int RW = ctx->mlp ? ctx->H : R;       // rows of the first (or only) weight matrix
     {   // every column in exactly one group
         std::vector<int> seen(D, 0);
         REQUIRE((int)ctx->h_gcols.size() == D, "groups cover %d columns but the data has %d", (int)ctx->h_gcols.size(), D);
@@ -672,15 +863,15 @@ int dks_fit(dks_ctx* ctx) {
     }
     TRY(dev_alloc(&ctx->d_bg, (size_t)N * D));
     TRY(dev_alloc(&ctx->d_wbg, (size_t)N));
-    TRY(dev_alloc(&ctx->d_W, (size_t)R * D));
-    TRY(dev_alloc(&ctx->d_b, (size_t)R));
+    TRY(dev_alloc(&ctx->d_W, (size_t)RW * D));
+    TRY(dev_alloc(&ctx->d_b, (size_t)RW));
     TRY(dev_alloc(&ctx->d_goff, (size_t)G + 1));
     TRY(dev_alloc(&ctx->d_gcols, (size_t)D));
     TRY(dev_alloc(&ctx->d_colmin, (size_t)D));
     TRY(dev_alloc(&ctx->d_colmax, (size_t)D));
     TRY(dev_alloc(&ctx->d_colnan, (size_t)D));
-    TRY(dev_alloc(&ctx->d_BW, (size_t)N * G * R));
-    TRY(dev_alloc(&ctx->d_scores, (size_t)N * R));
+    TRY(dev_alloc(&ctx->d_BW, (size_t)N * G * RW));
+    TRY(dev_alloc(&ctx->d_scores, (size_t)N * RW));
     TRY(dev_alloc(&ctx->d_Bbar, (size_t)G * R));
     TRY(dev_alloc(&ctx->d_fnull, (size_t)C));
     TRY(dev_alloc(&ctx->d_linkfnull, (size_t)C));
@@ -690,13 +881,35 @@ int dks_fit(dks_ctx* ctx) {
     cudaStream_t st = ctx->stream;
     CUDA_TRY(cudaMemcpyAsync(ctx->d_bg, ctx->h_bg.data(), sizeof(double) * N * D, cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(ctx->d_wbg, ctx->h_wbg.data(), sizeof(double) * N, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(ctx->d_W, ctx->h_W.data(), sizeof(double) * R * D, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(ctx->d_b, ctx->h_b.data(), sizeof(double) * R, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(ctx->d_W, ctx->h_W.data(), sizeof(double) * RW * D, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(ctx->d_b, ctx->h_b.data(), sizeof(double) * RW, cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(ctx->d_goff, ctx->h_goff.data(), sizeof(int32_t) * (G + 1), cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(ctx->d_gcols, ctx->h_gcols.data(), sizeof(int32_t) * D, cudaMemcpyHostToDevice, st));
 
     ctx->scale = (ctx->act == DKS_ACT_BINARY_LOGISTIC) ? -ctx->kappa * 1.4426950408889634
                : (ctx->act == DKS_ACT_SOFTMAX) ? 1.4426950408889634 : 1.0;
+    if (ctx->mlp) {
+        // BW1 [N][G][H] and base1 [N][H] by the linear fit kernels with W1 in place of W; fnull by a float64 forward
+        const int H = ctx->H;
+        TRY(dev_alloc(&ctx->d_W2, (size_t)R * H));
+        TRY(dev_alloc(&ctx->d_b2, (size_t)R));
+        CUDA_TRY(cudaMemcpyAsync(ctx->d_W2, ctx->h_W2.data(), sizeof(double) * R * H, cudaMemcpyHostToDevice, st));
+        CUDA_TRY(cudaMemcpyAsync(ctx->d_b2, ctx->h_b2.data(), sizeof(double) * R, cudaMemcpyHostToDevice, st));
+        if (ctx->mlp_hp > 0) {
+            TRY(dev_alloc(&ctx->d_mlp_perm, (size_t)ctx->mlp_hp));
+            TRY(dev_alloc(&ctx->d_mlp_w2abs, (size_t)ctx->mlp_hp));
+            CUDA_TRY(cudaMemcpyAsync(ctx->d_mlp_perm, ctx->h_mlp_perm.data(), sizeof(int) * ctx->mlp_hp, cudaMemcpyHostToDevice, st));
+            CUDA_TRY(cudaMemcpyAsync(ctx->d_mlp_w2abs, ctx->h_mlp_w2abs.data(), sizeof(float) * ctx->mlp_hp,
+                                     cudaMemcpyHostToDevice, st));
+        }
+        dks::fit_bw_kernel<<<cdiv((long long)N * G * H, 256), 256, 0, st>>>(ctx->d_bg, ctx->d_W, ctx->d_goff, ctx->d_gcols, N, D,
+                                                                               G, H, ctx->d_BW);
+        dks::fit_scores_kernel<<<cdiv((long long)N * H, 256), 256, 0, st>>>(ctx->d_BW, ctx->d_b, N, G, H, ctx->d_scores);
+        dks::fit_colstats_kernel<<<cdiv(D, 128), 128, 0, st>>>(ctx->d_bg, N, D, ctx->d_colmin, ctx->d_colmax, ctx->d_colnan);
+        dks::mlp::mlp_fnull_kernel<<<1, 32, 0, st>>>(ctx->d_scores, ctx->d_wbg, N, H, ctx->d_W2, ctx->d_b2, R, C, ctx->act,
+                                                     ctx->kappa, ctx->link, ctx->d_fnull, ctx->d_linkfnull);
+        ctx->launches += 4;
+    } else {
     dks::fit_bw_kernel<<<cdiv((long long)N * G * R, 256), 256, 0, st>>>(ctx->d_bg, ctx->d_W, ctx->d_goff, ctx->d_gcols, N, D,
                                                                            G, R, ctx->d_BW);
     dks::fit_scores_kernel<<<cdiv((long long)N * R, 256), 256, 0, st>>>(ctx->d_BW, ctx->d_b, N, G, R, ctx->d_scores);
@@ -706,6 +919,7 @@ int dks_fit(dks_ctx* ctx) {
     dks::fit_scale_kernel<<<cdiv((long long)N * G * R, 256), 256, 0, st>>>(ctx->d_BW, ctx->d_scores, ctx->d_wbg, N, G, R,
                                                                               ctx->scale, ctx->d_BWs, ctx->d_bases, ctx->d_wbf);
     ctx->launches += 5;
+    }
     CUDA_TRY(cudaGetLastError());
     ctx->h_fnull.resize(C);
     ctx->h_linkfnull.resize(C);
@@ -751,8 +965,12 @@ int dks_predict_host(dks_ctx* ctx, const double* X_host, int n, double* out_host
     TRY(dev_alloc(&dX, (size_t)n * ctx->D));
     TRY(dev_alloc(&dO, (size_t)n * ctx->C));
     CUDA_TRY(cudaMemcpyAsync(dX, X_host, sizeof(double) * n * ctx->D, cudaMemcpyHostToDevice, ctx->stream));
-    dks::predict_kernel<<<cdiv(n, 128), 128, 0, ctx->stream>>>(dX, ctx->d_W, ctx->d_b, n, ctx->D, ctx->R, ctx->C, ctx->act,
-                                                                ctx->kappa, dO);
+    if (ctx->mlp)
+        dks::mlp::mlp_predict_kernel<<<cdiv(n, 128), 128, 0, ctx->stream>>>(dX, ctx->d_W, ctx->d_b, ctx->d_W2, ctx->d_b2, n,
+                                                                             ctx->D, ctx->H, ctx->R, ctx->C, ctx->act, ctx->kappa, dO);
+    else
+        dks::predict_kernel<<<cdiv(n, 128), 128, 0, ctx->stream>>>(dX, ctx->d_W, ctx->d_b, n, ctx->D, ctx->R, ctx->C, ctx->act,
+                                                                    ctx->kappa, dO);
     ctx->launches += 1;
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(out_host, dO, sizeof(double) * n * ctx->C, cudaMemcpyDeviceToHost, ctx->stream));
@@ -829,7 +1047,39 @@ int dks_set_shared_plan(dks_ctx* ctx, int M, int S, const uint64_t* zbits_host, 
     memset(&pd, 0, sizeof(pd));
     pd.z = dz; pd.w = dw; pd.chol = dc; pd.ainv = di; pd.S = S; pd.W = W;
     pd.S_pad = (S + 31) / 32 * 32;
-    if (M == ctx->G && ctx->fitted && ctx->act == DKS_ACT_BINARY_LOGISTIC) {
+    if (M == ctx->G && ctx->fitted && ctx->act == DKS_ACT_BINARY_LOGISTIC && ctx->mlp) {
+        // MLP contexts: the solve tables of the shared-plan path and the plan's hidden part d'(s, j) (dks_mlp.cuh)
+        if (W == 1 && M - 1 <= dks::shared_path::PMAT_MAXK &&
+            dks::shared_path::wls_pmat_smem(M, pd.S_pad, false) + 8192 <= (size_t)ctx->max_smem_optin) {
+            float* pm = nullptr; double* dv = nullptr;
+            CUDA_TRY(cudaMalloc((void**)&pm, sizeof(float) * (size_t)(M - 1) * pd.S_pad));
+            CUDA_TRY(cudaMalloc((void**)&dv, sizeof(double) * (M - 1)));
+            ctx->plan_allocs[M].push_back(pm); ctx->plan_allocs[M].push_back(dv);
+            long long tot = (long long)(M - 1) * pd.S_pad;
+            dks::shared_path::plan_pmat_kernel<<<cdiv(tot, 256), 256, 0, ctx->stream>>>(dz, dw, di, S, pd.S_pad, M, pm);
+            dks::shared_path::plan_dvec_kernel<<<M - 1, 32, 0, ctx->stream>>>(dz, pm, S, pd.S_pad, M, dv);
+            ctx->launches += 2;
+            CUDA_TRY(cudaGetLastError());
+            pd.pmat = pm; pd.dvec = dv;
+        }
+        const int HP = ctx->mlp_hp, N = ctx->N;
+        if (HP > 0 && N <= dks::mlp::FAST_MAXN &&
+            dks::mlp::shared_smem_bytes(N, HP) <= (size_t)ctx->max_smem_optin &&
+            sizeof(float) * (size_t)M * HP <= (size_t)ctx->max_smem_optin) {
+            float* dT = nullptr; float* ld = nullptr;
+            CUDA_TRY(cudaMalloc((void**)&dT, sizeof(float) * (size_t)pd.S_pad * N * HP));
+            CUDA_TRY(cudaMalloc((void**)&ld, sizeof(float) * (size_t)pd.S_pad * N));
+            ctx->plan_allocs[M].push_back(dT); ctx->plan_allocs[M].push_back(ld);
+            const long long tot = (long long)pd.S_pad * N * HP, tl = (long long)pd.S_pad * N;
+            dks::mlp::mlp_plan_d_kernel<<<cdiv(tot, 256), 256, 0, ctx->stream>>>(dz, S, pd.S_pad, ctx->d_BW, ctx->d_scores, N, M,
+                                                                                ctx->H, HP, ctx->d_mlp_perm, ctx->d_mlp_w2abs, dT);
+            dks::mlp::mlp_plan_ld_kernel<<<cdiv(tl, 256), 256, 0, ctx->stream>>>(dz, S, pd.S_pad, ctx->d_BW, ctx->d_scores, N, M,
+                                                                                 ctx->H, ctx->d_W2, ld);
+            ctx->launches += 2;
+            CUDA_TRY(cudaGetLastError());
+            pd.mlp_dT = dT; pd.mlp_Ld = ld;
+        }
+    } else if (M == ctx->G && ctx->fitted && ctx->act == DKS_ACT_BINARY_LOGISTIC) {
         // shared-plan fast path: Dm table for the full varying set
         float* dm = nullptr;
         double* dme = nullptr;

@@ -30,6 +30,8 @@ struct PlanDev {
     const double* dvec64;  // [kpad] P z_L with the float64 P
     const double* ptw;     // [S_pad][kpw] float64 P^T supplied by the host for plans of more than 128 groups (dks_wide.cuh)
     const double* dvecw;   // [kpw] P z_L
+    const float* mlp_dT;   // [S_pad][N][HP] |W2|-scaled hidden part d'(s, j) of the full varying set (MLP shared-plan kernel)
+    const float* mlp_Ld;   // [S_pad][N] W2 . d(s, j)
     int kpw;
     int kpad;
     int S;
@@ -110,6 +112,23 @@ struct dks_ctx {
     float* dbg_T = nullptr;     // debug dump of the tcgen05 score tile of instance dbg_i ([dbg_rows][dbg_cols])
     int dbg_i = -1, dbg_rows = 0, dbg_cols = 0;
     float* dbg_time = nullptr;  // [6][256] clock64 timeline of CTA 0 (debug kernel variant)
+
+    // one-hidden-layer ReLU network (dks_set_mlp_model): d_W / d_b hold W1 [H x D] / b1 [H], R = output units;
+    // d_BW / d_scores hold BW1 [N][G][H] / base1 [N][H]
+    bool mlp = false;
+    int H = 0;
+    std::vector<double> h_W2, h_b2;
+    double *d_W2 = nullptr, *d_b2 = nullptr;
+    // shared-plan MLP kernel (binary head): unit order (positive W2 first, then negative, padded per chunk), HP = 0 when
+    // the padded width exceeds the kernel's 128 units
+    int mlp_hp = 0;
+    unsigned mlp_negmask = 0;
+    std::vector<int> h_mlp_perm;
+    std::vector<float> h_mlp_w2abs;
+    int* d_mlp_perm = nullptr;
+    float* d_mlp_w2abs = nullptr;
+    float* d_mlp_atab = nullptr;   // [QC][S_pad][HP] a'(q, s, u) of one chunk of instances
+    size_t cap_mlp_atab = 0;
 
     // host copies
     std::vector<double> h_bg, h_wbg, h_W, h_b;

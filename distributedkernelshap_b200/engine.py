@@ -15,7 +15,7 @@ import numpy as np
 from . import _cabi
 from .data import DenseData, convert_to_data, convert_to_link
 from .plan import build_plan, l1_tables, pack_dense_plan, projection, resolve_nsamples, sampling_info
-from .predictors import extract_linear_spec
+from .predictors import MLPModelSpec, extract_model_spec
 
 logger = logging.getLogger(__name__)
 
@@ -45,7 +45,8 @@ class GpuKernelExplainer:
     ----------
     model
         What the reference passes as ``predictor``: a bound ``predict_proba`` / ``decision_function`` of a linear
-        model, or a ``LinearModelSpec`` (see ``predictors.extract_linear_spec``).
+        model, ``predict_proba`` / ``predict`` of a one-hidden-layer ReLU ``MLPClassifier`` / ``MLPRegressor``, or a
+        ``LinearModelSpec`` / ``MLPModelSpec`` (see ``predictors.extract_model_spec``).
     data
         Background data: array, DataFrame or ``DenseData`` (groups and weights honoured).
     link
@@ -70,7 +71,8 @@ class GpuKernelExplainer:
         self.lib = _cabi.load()
         self.link = convert_to_link(link)
         self.model_callable = model
-        self.spec = extract_linear_spec(model)
+        self.spec = extract_model_spec(model)
+        self.is_mlp = isinstance(self.spec, MLPModelSpec)
         self.data = convert_to_data(data)
         if self.data.transposed:
             raise NotImplementedError("transposed DenseData (group sizes matching axis 0) is not supported")
@@ -78,8 +80,9 @@ class GpuKernelExplainer:
         if bg.ndim != 2:
             raise TypeError("background data must be two-dimensional")
         self.N, self.P = bg.shape
-        if self.spec.W.shape[1] != self.P:
-            raise ValueError(f"model expects {self.spec.W.shape[1]} columns, background has {self.P}")
+        n_cols = (self.spec.W1 if self.is_mlp else self.spec.W).shape[1]
+        if n_cols != self.P:
+            raise ValueError(f"model expects {n_cols} columns, background has {self.P}")
         if self.N > 100:
             logger.warning("Using %d background data samples could cause slower run times. Consider using "
                            "shap.sample(data, K) or shap.kmeans(data, K) to summarize the background as K samples.",
@@ -97,8 +100,13 @@ class GpuKernelExplainer:
         offsets[1:] = np.cumsum([len(g) for g in self.data.groups])
         cols = np.ascontiguousarray(np.concatenate([np.asarray(g, dtype=np.int32) for g in self.data.groups]), dtype=np.int32)
         _cabi.check(self.lib.dks_set_groups(self._ctx, _cabi.ptr(offsets), _cabi.ptr(cols), self.data.groups_size))
-        _cabi.check(self.lib.dks_set_model(self._ctx, _cabi.ptr(self.spec.W), _cabi.ptr(self.spec.b), self.spec.W.shape[0],
-                                           self.spec.act_code, self.spec.kappa, int(self.spec.scalar_out)))
+        if self.is_mlp:
+            sp = self.spec
+            _cabi.check(self.lib.dks_set_mlp_model(self._ctx, _cabi.ptr(sp.W1), _cabi.ptr(sp.b1), sp.W1.shape[0], _cabi.ptr(sp.W2),
+                                                   _cabi.ptr(sp.b2), sp.W2.shape[0], sp.act_code, sp.kappa, int(sp.scalar_out)))
+        else:
+            _cabi.check(self.lib.dks_set_model(self._ctx, _cabi.ptr(self.spec.W), _cabi.ptr(self.spec.b), self.spec.W.shape[0],
+                                               self.spec.act_code, self.spec.kappa, int(self.spec.scalar_out)))
         link_code = _cabi.LINK_LOGIT if str(self.link) == "logit" else _cabi.LINK_IDENTITY
         _cabi.check(self.lib.dks_set_link(self._ctx, link_code))
         self.set_kernel(kernel)
@@ -122,13 +130,14 @@ class GpuKernelExplainer:
 
     # ------------------------------------------------------------------------------------------------------
     def _check_model_against_callable(self, bg):
-        """The extracted linear model must reproduce the user's callable on the background rows."""
+        """The extracted model must reproduce the user's callable on the background rows (GPU float64 forward)."""
         if not callable(self.model_callable):
             return
         want = np.asarray(self.model_callable(bg), dtype=np.float64).reshape(self.N, -1)
         got = self.predict(bg)
         if want.shape != got.shape or not np.allclose(got, want, rtol=1e-7, atol=1e-9, equal_nan=True):
-            raise ValueError("the linear model extracted from `predictor` does not reproduce predictor(background): "
+            raise ValueError(f"the {'network' if self.is_mlp else 'linear model'} extracted from `predictor` does not "
+                             "reproduce predictor(background): "
                              "refusing to explain a different function (max abs diff "
                              f"{np.max(np.abs(got - want)) if want.shape == got.shape else 'shape mismatch'})")
 
@@ -142,6 +151,9 @@ class GpuKernelExplainer:
     def set_kernel(self, kernel):
         code = {"auto": _cabi.KERNEL_AUTO, "simt": _cabi.KERNEL_SIMT, "tcgen05": _cabi.KERNEL_TCGEN05,
                 "shared": _cabi.KERNEL_SHARED}[kernel]
+        if kernel == "tcgen05" and getattr(self, "is_mlp", False):
+            raise NotImplementedError("the tcgen05 kernel evaluates linear models only; networks run on 'auto', 'shared' "
+                                      "or 'simt'")
         _cabi.check(self.lib.dks_set_kernel(self._ctx, code))
         self.kernel = kernel
 

@@ -1,4 +1,4 @@
-"""The model side of the hot path: linear scores followed by a probability head.
+"""The model side of the hot path: linear scores (or one hidden layer of ReLU units) followed by a probability head.
 
 The reference passes an opaque Python callable (``clf.predict_proba`` of a scikit-learn
 ``LogisticRegression(multi_class='multinomial')``, benchmarks/ray_pool.py:34, scripts/fit_adult_model.py:27-32).
@@ -121,3 +121,99 @@ def extract_linear_spec(predictor):
             raise TypeError("classifier.predict returns labels, which KernelSHAP cannot explain; pass predict_proba")
         return LinearModelSpec(coef, intercept, "identity", scalar_out=coef.shape[0] == 1)
     raise TypeError(f"unsupported predictor method {method!r}")
+
+
+MLP_MAX_HIDDEN = 128
+MLP_MAX_OUTPUTS = 8
+
+
+class MLPModelSpec:
+    """One hidden layer of ReLU units, then a head: ``h = relu(X W1^T + b1)``, ``z = h W2^T + b2``.  ``W1`` is [H, D],
+    ``b1`` [H], ``W2`` [R, H], ``b2`` [R]; ``activation`` / ``kappa`` / ``scalar_out`` as in ``LinearModelSpec``
+    ('binary_logistic' is scikit-learn's logistic output unit with kappa = 1: outputs [1 - s, s])."""
+
+    def __init__(self, W1, b1, W2, b2, activation, kappa=1.0, scalar_out=False):
+        self.W1 = np.ascontiguousarray(np.atleast_2d(np.asarray(W1, dtype=np.float64)))
+        self.b1 = np.ascontiguousarray(np.atleast_1d(np.asarray(b1, dtype=np.float64)))
+        self.W2 = np.ascontiguousarray(np.atleast_2d(np.asarray(W2, dtype=np.float64)))
+        self.b2 = np.ascontiguousarray(np.atleast_1d(np.asarray(b2, dtype=np.float64)))
+        H, R = self.W1.shape[0], self.W2.shape[0]
+        if self.b1.shape != (H,):
+            raise ValueError(f"W1 has {H} rows but b1 has {self.b1.shape[0]} entries")
+        if self.W2.shape[1] != H:
+            raise ValueError(f"W2 has {self.W2.shape[1]} columns but the hidden layer has {H} units")
+        if self.b2.shape != (R,):
+            raise ValueError(f"W2 has {R} rows but b2 has {self.b2.shape[0]} entries")
+        if activation not in ("identity", "binary_logistic", "softmax"):
+            raise ValueError(f"unknown activation {activation!r}")
+        if activation == "binary_logistic" and R != 1:
+            raise ValueError("binary_logistic needs a single output unit")
+        if activation == "softmax" and R < 2:
+            raise ValueError("softmax needs at least two output units")
+        if H > MLP_MAX_HIDDEN:
+            raise NotImplementedError(f"{H} hidden units: the CUDA engine handles at most {MLP_MAX_HIDDEN}")
+        if R > MLP_MAX_OUTPUTS:
+            raise NotImplementedError(f"{R} output units: the CUDA engine handles at most {MLP_MAX_OUTPUTS}")
+        self.activation = activation
+        self.kappa = float(kappa)
+        self.scalar_out = bool(scalar_out)
+
+    act_code = LinearModelSpec.act_code
+
+    @property
+    def n_outputs(self):
+        return 2 if self.activation == "binary_logistic" else self.W2.shape[0]
+
+    @property
+    def n_features(self):
+        return self.W1.shape[1]
+
+    def __call__(self, X):
+        """NumPy float64 forward with scikit-learn's conventions."""
+        X = np.asarray(X, dtype=np.float64)
+        if X.ndim == 1:
+            X = X.reshape(1, -1)
+        h = np.maximum(X @ self.W1.T + self.b1, 0.0)
+        return LinearModelSpec(self.W2, self.b2, self.activation, self.kappa, self.scalar_out)(h)
+
+
+def _mlp_spec_from_sklearn(owner, method):
+    """``MLPClassifier.predict_proba`` / ``MLPRegressor.predict`` of a fitted one-hidden-layer ReLU network."""
+    coefs, intercepts = owner.coefs_, owner.intercepts_
+    if len(coefs) != 2:
+        raise NotImplementedError(f"{type(owner).__name__} has {len(coefs) - 1} hidden layers: the CUDA engine explains "
+                                  "networks of one hidden layer")
+    if owner.activation != "relu":
+        raise NotImplementedError(f"hidden activation {owner.activation!r}: the CUDA engine explains ReLU networks only")
+    out = owner.out_activation_
+    W1, b1 = np.asarray(coefs[0], dtype=np.float64).T, intercepts[0]
+    W2, b2 = np.asarray(coefs[1], dtype=np.float64).T, intercepts[1]
+    if hasattr(owner, "classes_"):
+        if method != "predict_proba":
+            raise TypeError("classifier.predict returns labels, which KernelSHAP cannot explain; pass predict_proba")
+        if out == "logistic" and W2.shape[0] == 1:
+            return MLPModelSpec(W1, b1, W2, b2, "binary_logistic", kappa=1.0)
+        if out == "softmax":
+            return MLPModelSpec(W1, b1, W2, b2, "softmax")
+        raise NotImplementedError(f"{type(owner).__name__} with {W2.shape[0]} {out} outputs (multilabel): only binary "
+                                  "and multi-class heads are supported")
+    if method != "predict":
+        raise TypeError(f"unsupported predictor method {method!r}")
+    if out != "identity":
+        raise NotImplementedError(f"regression output activation {out!r} is not supported")
+    return MLPModelSpec(W1, b1, W2, b2, "identity", scalar_out=W2.shape[0] == 1)
+
+
+def _is_sklearn_mlp(owner):
+    return all(hasattr(owner, a) for a in ("coefs_", "intercepts_", "activation", "out_activation_"))
+
+
+def extract_model_spec(predictor):
+    """What the engine calls: an ``MLPModelSpec`` for an ``MLPModelSpec`` or a bound ``predict_proba`` / ``predict`` of a
+    fitted scikit-learn ``MLPClassifier`` / ``MLPRegressor``; ``extract_linear_spec(predictor)`` for everything else."""
+    if isinstance(predictor, MLPModelSpec):
+        return predictor
+    owner = getattr(predictor, "__self__", None)
+    if owner is not None and _is_sklearn_mlp(owner):
+        return _mlp_spec_from_sklearn(owner, getattr(predictor, "__name__", None))
+    return extract_linear_spec(predictor)

@@ -45,7 +45,7 @@ extern "C" {
 #define DKS_LINK_IDENTITY 0
 #define DKS_LINK_LOGIT 1
 
-/* which fused kernel evaluates the coalitions */
+/* which fused kernel evaluates the coalitions (on a context set up with dks_set_mlp_model: see there) */
 #define DKS_KERNEL_AUTO 0
 #define DKS_KERNEL_SIMT 1       /* CUDA-core kernel (all shapes) */
 #define DKS_KERNEL_TCGEN05 2    /* tensor-core kernel: Z tile x background tile on tcgen05/TMEM */
@@ -77,6 +77,15 @@ int dks_set_groups(dks_ctx* ctx, const int32_t* group_offsets, const int32_t* gr
  * DKS_ACT_BINARY_LOGISTIC only.  scalar_out != 0 marks a predictor returning a 1-D array (vector_out False). */
 int dks_set_model(dks_ctx* ctx, const double* W_host, const double* b_host, int R, int activation, double kappa,
                   int scalar_out);
+/* instead of dks_set_model: a network of one hidden layer of H ReLU units (scikit-learn MLPClassifier / MLPRegressor with
+ * activation='relu'), scores z = W2 relu(W1 x + b1) + b2 with W1 [H x D] and W2 [R x H] row-major, b1 [H], b2 [R]; the head
+ * (activation, kappa, scalar_out) as in dks_set_model.  H <= 128, R <= 8; at most 64 groups (DKS_ERR_UNSUPPORTED beyond).
+ * Kernels on such a context: DKS_KERNEL_AUTO = shared-plan MLP kernel for the instances whose groups all vary (binary head,
+ * uniform background weights, plans of the engine) and the general MLP kernel for the rest; DKS_KERNEL_SHARED the same, but
+ * DKS_ERR_UNSUPPORTED where the shared-plan kernel does not apply; DKS_KERNEL_SIMT the general MLP kernel for every instance;
+ * DKS_KERNEL_TCGEN05 is unsupported. */
+int dks_set_mlp_model(dks_ctx* ctx, const double* W1_host, const double* b1_host, int H, const double* W2_host,
+                      const double* b2_host, int R, int activation, double kappa, int scalar_out);
 int dks_set_link(dks_ctx* ctx, int link);
 /* runs the fit kernels (grouped background scores, fnull = sum_j w_j f(bg_j), link(fnull)); synchronises. */
 int dks_fit(dks_ctx* ctx);
